@@ -2,7 +2,7 @@
 """bench.py -- committed ops/s of the replication hot path (BASELINE.json metric:
 "committed ops/s and p50/p99 commit latency, 64B reqs, 5 replicas").
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A *step* is one pass of the hot path over one batch of synthetic requests:
 `--batch` SEND requests of `--payload` bytes are appended to the leader's log,
@@ -80,6 +80,8 @@ def parse():
     ap.add_argument("--leader-ctas", type=int, default=16, help="leader worker CTAs (SMs building tiles in parallel)")
     ap.add_argument("--spread", action="store_true",
                     help="single process: place replica r on GPU r %% visible GPUs (NVLink path)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step committed as DIR/<name>.npy (see dump_outputs)")
     return ap.parse_args()
 
 
@@ -544,6 +546,8 @@ def run_ours(args):
     off = cell.leader.offsets()
     # every replica this rank hosts holds the leader's live log (size-independent property of the timed run itself)
     live = live_log_check(cell, dist, gloo, rank, world, n, L) if not args.no_parity else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(cell, args.dump_outputs, req - 1, st["tickets_committed"], payload)
     cell.close()
 
     # =========================== e2e: host buffers through the C ABI =====================
@@ -804,6 +808,39 @@ def live_log_check(cell, dist, gloo, rank, world, n, L):
     return {"followers_equal_leader": bool(ok), "entries_compared_per_replica": int(allr[0]["tail_entries"]) if allr else 0,
             "what": "after the timed multi-lap run: the newest entries of every replica's live log (reply bytes masked), end, commit "
                     "and last idx equal within each group; entries parse with consecutive idx from head to end"}
+
+
+def dump_outputs(cell, directory, last_req, committed, payload):
+    """What the timed path hands its caller, for comparing two builds output for output: every hosted replica's copy of
+    the newest requests of the last step (a step is larger than the log ring, so only its newest requests are still
+    live; at most 4096 of them, and at most 64 MiB in all), and the number of committed tickets.
+
+      requests.npy           float64 [replica, request, (term, req_id, connection, type, sender)]
+      payloads.npy           float32 [replica, request, byte]
+      tickets_committed.npy  float64 [1]
+
+    Left out: the entry's idx, which counts the HEAD entries the pruning rule interleaves at timing-dependent places, the
+    reply bytes (acks, also timing) and padding (whatever an earlier lap of the ring left there)."""
+    import orc as O
+    os.makedirs(directory, exist_ok=True)
+    count = max(1, min(4096, (64 << 20) // ((4 * payload + 40) * len(cell.local))))
+    reqs, pays = [], []
+    for r in cell.local:
+        o = r.offsets()
+        img = r.image()
+        ents = O.walk_entries(img, o["head"], o["end"], cell.L) if o["end"] != cell.L else []
+        sends = [e for e, _ in ents if img[e + 26] == SEND][-count:]
+        hdr = np.stack([img[e:e + 28] for e in sends]) if sends else np.zeros((0, 28), np.uint8)
+        fields = np.stack([hdr[:, 8:16].copy().view("<u8")[:, 0], hdr[:, 16:24].copy().view("<u8")[:, 0],
+                           hdr[:, 24:26].copy().view("<u2")[:, 0], hdr[:, 26], hdr[:, 27]], axis=1).astype(np.float64)
+        if fields[:, 1].tolist() != list(range(last_req - count + 1, last_req + 1)):
+            raise SystemExit(f"--dump-outputs: replica {r.idx} does not hold the newest {count} requests "
+                             f"(found {len(sends)}, expected req_ids up to {last_req})")
+        reqs.append(fields)
+        pays.append(np.stack([img[e + 50:e + 50 + payload] for e in sends]).astype(np.float32))
+    np.save(os.path.join(directory, "requests.npy"), np.stack(reqs))
+    np.save(os.path.join(directory, "payloads.npy"), np.stack(pays))
+    np.save(os.path.join(directory, "tickets_committed.npy"), np.array([committed], dtype=np.float64))
 
 
 def proxy_closed_loop_leg(args, n, payload, log, conns=16, nreq=20000, steps=3):

@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Generate tests/golden/refstack_golden.json from the RUNNING REFERENCE: the reference's unmodified election /
+"""Generate tests/golden/refstack_golden.json and refstack_runs_golden.json from the RUNNING REFERENCE: the reference's unmodified election /
 replication / commit code and proxy.c (oracle/_ref/libref_stack.so on oracle/verbs_shim, built from /root/reference
 by oracle/build_refapp.sh) execute each scenario as N processes; the fixture records, per replica, the offsets and
 the SHA-256 of the log it left behind (leader: all bytes; followers: reply[0..12] masked, the H5 rule of SURVEY.md
@@ -8,7 +8,8 @@ s8c), with the leader index and term the election produced.  Run where /root/ref
     python tests/golden/gen_refstack_golden.py
 
 tests/test_golden.py replays the same streams through the oracle (anywhere) and tests/test_gpu_parity.py through the
-CUDA engine (GPU box) and compares against these hashes."""
+CUDA engine and compares against these hashes; tests/test_oracle_vs_refstack.py compares the oracle with the runs
+recorded in refstack_runs_golden.json."""
 import hashlib
 import json
 import os
@@ -17,8 +18,10 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE))
 
-import orc as O          # noqa: E402
-import refstack as R     # noqa: E402
+import orc as O                          # noqa: E402
+import refgold                           # noqa: E402
+import refstack as R                     # noqa: E402
+import test_oracle_vs_refstack as TVS    # noqa: E402
 
 SCENARIOS = [dict(name="ref3_2conn_300x64", n=3, nconn=2, nreq=300, plen=64),
              dict(name="ref5_3conn_200x128", n=5, nconn=3, nreq=200, plen=128),
@@ -48,3 +51,6 @@ if __name__ == "__main__":
         json.dump(dict(source="oracle/_ref/libref_stack.so: reference src/dare/*.c + proxy.c, unmodified, on oracle/verbs_shim",
                        scenarios=out), f, indent=1, sort_keys=True)
     print("wrote", path)
+    refgold.write("refstack_runs_golden.json", "oracle/_ref/libref_stack.so: reference src/dare/*.c + proxy.c, unmodified "
+                  "(commit 896959f), on oracle/verbs_shim", TVS.record())
+    print("wrote refstack_runs_golden.json")

@@ -3,12 +3,13 @@ election / replication / commit code (oracle/_ref/libref_stack.so on the verbs s
 engine (through the C ABI) are fed the same request stream; the logs they leave behind must be identical --
 leader copy: every byte, reply bytes included; follower copies: every byte outside reply[0..12] (H5 mask,
 SURVEY.md s8c) plus the follower's own ack byte (I7).  Leader index and term are whatever the reference's
-election produced."""
-import numpy as np
+election produced.  The reference's side is the recording of these runs in tests/golden/refstack_runs_golden.json
+(tests/golden/gen_refstack_golden.py), which tests/test_oracle_vs_refstack.py also checks the oracle against."""
 import pytest
 
 import orc as O
 import refstack as R
+from refgold import recorded, sha
 
 pytestmark = [pytest.mark.gpu, pytest.mark.timeout(300)]
 
@@ -25,14 +26,7 @@ def eng():
 
 @pytest.mark.parametrize("n,nconn,nreq,plen", [(3, 2, 300, 64), (5, 3, 200, 128), (3, 1, 120, -3000), (7, 4, 400, 64)])
 def test_engine_log_equals_reference_log(eng, n, nconn, nreq, plen):
-    if not R.available():
-        pytest.skip("oracle/_ref/libref_stack.so absent (built only where /root/reference exists)")
-    try:
-        rr = R.run(n, nconn, nreq, plen, prune=1000.0)
-    except RuntimeError as e:
-        # the reference stack needs process_vm_writev between sibling processes; a box that forbids it cannot host the
-        # CPU side of this comparison (the golden vectors of the same runs still apply: test_gpu_parity.py)
-        pytest.skip(f"the reference stack could not run on this box: {str(e)[:200]}")
+    rr = recorded("refstack_runs_golden.json")[f"log_equals/{n}/{nconn}/{nreq}/{plen}"]
     lead, term = rr["leader"], rr["term"]
     nd = eng.lib().apus_device_count()
     with eng.Group(n, devices=[i % nd for i in range(n)], leader=lead, term=term, log_size=O.LOG_SIZE) as g:
@@ -46,13 +40,14 @@ def test_engine_log_equals_reference_log(eng, n, nconn, nreq, plen):
             if i == lead:
                 assert eo["tail"] == ro["tail"]
             got, want = g.replicas[i].image(0, end), rr["images"][i]
-            ents = O.walk_entries(want, 0, end, O.LOG_SIZE)
+            assert want["len"] == end
+            ents = O.walk_entries(got, 0, end, O.LOG_SIZE)
+            assert len(ents) == rr["entries"]
             if i != lead:
                 for off, _ in ents:
-                    assert got[off + 28 + i] == 1 and want[off + 28 + i] == 1
-                got, want = O.mask_replies(got, ents), O.mask_replies(want, ents)
-            if not np.array_equal(got, want):
-                dd = np.nonzero(got != want)[0]
-                raise AssertionError(f"replica {i} (leader {lead}, term {term}): {len(dd)} bytes differ from the reference, "
-                                     f"first at {int(dd[0])}: engine {got[dd[0]]} reference {want[dd[0]]}")
+                    assert got[off + 28 + i] == 1
+                assert all(bytes.fromhex(k)[1 + i] == 1 for k in want["stamps"])
+                assert sha(O.mask_replies(got, ents)) == want["masked_sha"], f"replica {i} (leader {lead}, term {term})"
+            else:
+                assert sha(got) == want["sha"], f"replica {i} (leader {lead}, term {term})"
         assert g.leader.committed() == len(ents)

@@ -1,144 +1,148 @@
-"""The restated oracle (oracle/orc_log.h, cluster_sim.inc) against the compiled
-reference header (oracle/_ref, built from /root/reference/src/include/dare/dare_log.h).
+"""The restated oracle (oracle/orc_log.h, cluster_sim.inc) against the compiled reference header (dare_log.h,
+unmodified, built into oracle/_ref by oracle/Makefile).
 
-These tests only run where the reference tree exists (this container); on the GPU
-box the same restatement is pinned by tests/golden/ instead (test_golden.py).
+What the reference produced for every scenario below is recorded in tests/golden/ref_log_golden.json
+(tests/golden/gen_golden.py re-records it where the reference's sources exist), so these tests run anywhere.
+Each `observe_*` function is run on the reference by the generator and on the oracle by the test.
 """
 import numpy as np
 import pytest
 
 import orc as O
 import streams as S
+from refgold import digest, recorded
+
+GOLD = "ref_log_golden.json"
 
 
-def play(oracle, stream, length, term=1, pre=None):
-    log = O.Log(oracle, length)
-    if pre:
-        pre(log)
-    rets = []
-    for typ, clt, rid, payload in stream:
-        rets.append(log.append(term, rid, clt, typ, O.cmd_image(payload)))
-    return log, rets
+def reference(key):
+    return recorded(GOLD)[key]
 
 
-def same_log(a: O.Log, b: O.Log):
-    oa, ob = a.offsets(), b.offsets()
-    assert oa == ob
-    ia, ib = a.image(), b.image()
-    assert np.array_equal(ia, ib), f"first diff at {int(np.argmax(ia != ib))}"
+def observe_layout(ref):
+    return dict(sizeof_entry=int(ref.sizeof_entry()), sizeof_log=int(ref.lib.ref_sizeof_log()),
+                log_size=int(ref.lib.ref_log_size()))
 
 
-def test_layout_constants(ref):
-    assert ref.sizeof_entry() == 64
-    assert ref.lib.ref_sizeof_log() == 319656
-    assert ref.lib.ref_log_size() == O.LOG_SIZE
+def test_layout_constants(orc):
+    g = reference("layout")
+    assert g == dict(sizeof_entry=64, sizeof_log=319656, log_size=O.LOG_SIZE)
+    assert orc.sizeof_entry() == g["sizeof_entry"]
 
 
-def test_kat_from_survey(ref, orc):
-    """SURVEY.md s8c known-answer vector, re-generated from the compiled reference."""
-    orc.set_rules(O.RULES_REFERENCE)
+KAT = [(1, 0, 128), (2, 128, 256), (3, 256, 384), (4, 384, 548), (5, 548, 4708), (6, 4708, 4772), (7, 4772, 4836)]
+
+
+def observe_kat(oracle):
+    oracle.set_rules(O.RULES_REFERENCE)
     lens = [64, 64, 64, 100, 4096]
-    expect = [(1, 0, 128), (2, 128, 256), (3, 256, 384), (4, 384, 548), (5, 548, 4708),
-              (6, 4708, 4772), (7, 4772, 4836)]
-    for oracle in (ref, orc):
-        log = O.Log(oracle)
-        off = log.offsets()
-        assert (off["head"], off["apply"], off["commit"]) == (0, 0, 0)
-        assert off["end"] == off["tail"] == off["len"] == 67108864
-        got = []
-        for i, ln in enumerate(lens):
-            idx = log.append(1, i + 1, 0x0100, O.SEND, O.cmd_image(S.payload_kat(i, ln)))
+    log = O.Log(oracle)
+    off = log.offsets()
+    first = [off[k] for k in ("head", "apply", "commit", "end", "tail", "len")]
+    got = []
+    for i, ln in enumerate(lens):
+        idx = log.append(1, i + 1, 0x0100, O.SEND, O.cmd_image(S.payload_kat(i, ln)))
+        o = log.offsets()
+        got.append((idx, o["tail"], o["end"]))
+    idx = log.append(1, 6, 0x0100, O.CONNECT, O.cmd_image(b""))
+    o = log.offsets(); got.append((idx, o["tail"], o["end"]))
+    idx = log.append(1, 7, 0x0100, O.NOOP, b"")
+    o = log.offsets(); got.append((idx, o["tail"], o["end"]))
+    fnv = O.fnv1a(log.image(0, 4836))
+    log.close()
+    return dict(first=first, got=got, fnv=f"{fnv:016x}")
+
+
+def test_kat_from_survey(orc):
+    """SURVEY.md s8c known-answer vector, as the compiled reference produced it."""
+    g = reference("kat")
+    # (idx, tail, end) are the triples quoted in SURVEY.md s8c.  The FNV-1a-64 quoted there came from a probe harness
+    # that was never committed and cannot be reproduced byte for byte; this checksum is the compiled reference's.
+    assert g == dict(first=[0, 0, 0, 67108864, 67108864, 67108864], got=[list(t) for t in KAT], fnv="6ef37439cde8f856")
+    assert digest(observe_kat(orc)) == g
+
+
+def observe_random_stream(oracle, seed, length):
+    oracle.set_rules(O.RULES_REFERENCE)
+    stream = S.ragged_stream(600, 300, conns=3, seed=seed, close_every=50)
+    log = O.Log(oracle, length)
+    rets = []
+    r = np.random.default_rng(seed + 99)
+    for k, (typ, clt, rid, payload) in enumerate(stream):
+        rets.append(log.append(1 + k // 200, rid, clt, typ, O.cmd_image(payload)))
+        # advance head now and then so the ring keeps accepting entries
+        if k % 7 == 0:
             o = log.offsets()
-            got.append((idx, o["tail"], o["end"]))
-        idx = log.append(1, 6, 0x0100, O.CONNECT, O.cmd_image(b""))
-        o = log.offsets(); got.append((idx, o["tail"], o["end"]))
-        idx = log.append(1, 7, 0x0100, O.NOOP, b"")
-        o = log.offsets(); got.append((idx, o["tail"], o["end"]))
-        assert got == expect
-        # (idx, tail, end) above are the triples quoted in SURVEY.md s8c.  The FNV-1a-64
-        # quoted there came from a probe harness that was never committed and cannot be
-        # reproduced byte for byte; this checksum is regenerated from the compiled
-        # reference header (oracle/_ref) and pinned in tests/golden/ as well.
-        assert O.fnv1a(log.image(0, 4836)) == 0x6EF37439CDE8F856
-        log.close()
+            if o["end"] != o["len"]:
+                log.set_offsets(head=o["tail"], apply=o["tail"], commit=o["tail"])
+        if r.random() < 0.05:
+            rets.append(log.append(1, 0, 0, O.NOOP, b""))
+        if r.random() < 0.03:
+            rets.append(log.append(1, 0, 0, O.CONFIG, O.cid_image(3)))
+        if r.random() < 0.03:
+            rets.append(log.append(1, 0, 0, O.HEAD, (12345).to_bytes(8, "little")))
+    out = dict(rets=rets, offsets=log.offsets(), image=log.image())
+    log.close()
+    return out
+
+
+RANDOM_STREAMS = [(seed, length) for length in (4096, 1 << 16) for seed in (1, 2, 3)]
 
 
 @pytest.mark.parametrize("seed", [1, 2, 3])
 @pytest.mark.parametrize("length", [4096, 1 << 16])
-def test_random_streams_with_wraps(ref, orc, seed, length):
+def test_random_streams_with_wraps(orc, seed, length):
     """Small rings force every wrap rule of log_append_entry (ghost header, header
     does not fit, exact fit, full) -- reference rules must match bit for bit."""
-    orc.set_rules(O.RULES_REFERENCE)
-    stream = S.ragged_stream(600, 300, conns=3, seed=seed, close_every=50)
-    rng = np.random.default_rng(seed)
-
-    def run(oracle):
-        log = O.Log(oracle, length)
-        rets = []
-        r = np.random.default_rng(seed + 99)
-        for k, (typ, clt, rid, payload) in enumerate(stream):
-            rets.append(log.append(1 + k // 200, rid, clt, typ, O.cmd_image(payload)))
-            # advance head now and then so the ring keeps accepting entries
-            if k % 7 == 0:
-                o = log.offsets()
-                if o["end"] != o["len"]:
-                    log.set_offsets(head=o["tail"], apply=o["tail"], commit=o["tail"])
-            if r.random() < 0.05:
-                rets.append(log.append(1, 0, 0, O.NOOP, b""))
-            if r.random() < 0.03:
-                rets.append(log.append(1, 0, 0, O.CONFIG, O.cid_image(3)))
-            if r.random() < 0.03:
-                rets.append(log.append(1, 0, 0, O.HEAD, (12345).to_bytes(8, "little")))
-        return log, rets
-
-    la, ra = run(ref)
-    lb, rb = run(orc)
-    assert ra == rb
-    same_log(la, lb)
-    la.close(); lb.close()
+    assert digest(observe_random_stream(orc, seed, length)) == reference(f"random_stream/{seed}/{length}")
 
 
-@pytest.mark.parametrize("left", [0, 1, 40, 63, 64, 65, 100, 127, 128, 129, 200])
-@pytest.mark.parametrize("typ", [O.SEND, O.NOOP, O.HEAD, O.CONFIG])
-def test_wrap_edges(ref, orc, left, typ):
+def observe_wrap_edge(oracle, left, typ):
     """Place `end` exactly `left` bytes before len and append one entry (64 B payload)."""
-    orc.set_rules(O.RULES_REFERENCE)
+    oracle.set_rules(O.RULES_REFERENCE)
     length = 8192
-    res = []
-    for oracle in (ref, orc):
-        log = O.Log(oracle, length)
-        # fill with 64 B NOOP-size strides up to the desired position, head moved away
-        log.append(1, 1, 7, O.SEND, O.cmd_image(b"x" * 64))
-        pos = length - left
-        log.poke(0, bytes(range(256)) * (length // 256))      # stale bytes everywhere
-        # fabricate a log whose last entry ends at pos: tail entry must parse
-        tail = pos - 64
-        hdr = (41).to_bytes(8, "little") + (1).to_bytes(8, "little") + bytes(8) + bytes([7, 0, O.NOOP, 0]) + bytes(36)
-        log.poke(tail, hdr)
-        log.set_offsets(head=256, apply=256, commit=256, end=pos, tail=tail, old_end=pos)
-        data = {O.SEND: O.cmd_image(bytes(range(64))), O.NOOP: b"", O.HEAD: (77).to_bytes(8, "little"),
-                O.CONFIG: O.cid_image(5)}[typ]
-        idx = log.append(2, 9, 0x0203, typ, data)
-        res.append((idx, log.offsets(), log.image()))
-        log.close()
-    assert res[0][0] == res[1][0]
-    assert res[0][1] == res[1][1]
-    assert np.array_equal(res[0][2], res[1][2])
+    log = O.Log(oracle, length)
+    # fill with 64 B NOOP-size strides up to the desired position, head moved away
+    log.append(1, 1, 7, O.SEND, O.cmd_image(b"x" * 64))
+    pos = length - left
+    log.poke(0, bytes(range(256)) * (length // 256))      # stale bytes everywhere
+    # fabricate a log whose last entry ends at pos: tail entry must parse
+    tail = pos - 64
+    hdr = (41).to_bytes(8, "little") + (1).to_bytes(8, "little") + bytes(8) + bytes([7, 0, O.NOOP, 0]) + bytes(36)
+    log.poke(tail, hdr)
+    log.set_offsets(head=256, apply=256, commit=256, end=pos, tail=tail, old_end=pos)
+    data = {O.SEND: O.cmd_image(bytes(range(64))), O.NOOP: b"", O.HEAD: (77).to_bytes(8, "little"),
+            O.CONFIG: O.cid_image(5)}[typ]
+    idx = log.append(2, 9, 0x0203, typ, data)
+    out = dict(idx=idx, offsets=log.offsets(), image=log.image())
+    log.close()
+    return out
 
 
-def test_wrap_into_head_zero_is_full(ref, orc):
+WRAP_LEFT = [0, 1, 40, 63, 64, 65, 100, 127, 128, 129, 200]
+WRAP_TYPES = [O.SEND, O.NOOP, O.HEAD, O.CONFIG]
+
+
+@pytest.mark.parametrize("left", WRAP_LEFT)
+@pytest.mark.parametrize("typ", WRAP_TYPES)
+def test_wrap_edges(orc, left, typ):
+    assert digest(observe_wrap_edge(orc, left, typ)) == reference(f"wrap_edge/{left}/{typ}")
+
+
+def observe_wrap_into_head_zero(oracle):
+    oracle.set_rules(O.RULES_REFERENCE)
+    log = O.Log(oracle, 4096)
+    rets = [log.append(1, i + 1, 1, O.SEND, O.cmd_image(b"a" * 70)) for i in range(40)]
+    out = dict(rets=rets, offsets=log.offsets(), image=log.image())
+    log.close()
+    return out
+
+
+def test_wrap_into_head_zero_is_full(orc):
     """H11(iii): wrapping while head == 0 reports full and leaves end = 0."""
-    orc.set_rules(O.RULES_REFERENCE)
-    out = []
-    for oracle in (ref, orc):
-        log = O.Log(oracle, 4096)
-        rets = [log.append(1, i + 1, 1, O.SEND, O.cmd_image(b"a" * 70)) for i in range(40)]
-        out.append((rets, log.offsets(), log.image()))
-        log.close()
-    assert out[0][0] == out[1][0]
-    assert out[0][1] == out[1][1]
-    assert np.array_equal(out[0][2], out[1][2])
-    assert 0 in out[0][0]
+    got = observe_wrap_into_head_zero(orc)
+    assert digest(got) == reference("wrap_into_head_zero")
+    assert 0 in got["rets"]
 
 
 def cluster_script(oracle, n, stream, length, schedule_seed):
@@ -180,54 +184,67 @@ def cluster_script(oracle, n, stream, length, schedule_seed):
     return obs
 
 
-@pytest.mark.parametrize("n", [1, 3, 5, 7])
-def test_cluster_steps_match(ref, orc, n):
-    orc.set_rules(O.RULES_REFERENCE)
+def observe_cluster_steps(oracle, n):
+    oracle.set_rules(O.RULES_REFERENCE)
     stream = S.ragged_stream(400, 200, conns=4, seed=n, close_every=40)
-    a = cluster_script(ref, n, stream, 1 << 20, 5)
-    b = cluster_script(orc, n, stream, 1 << 20, 5)
-    assert a["offsets"] == b["offsets"]
-    assert a["applied"] == b["applied"]
-    assert a["commits"] == b["commits"]
-    assert a["store"] == b["store"] and a["update_state"] == b["update_state"]
-    assert a["bytes_rep"] == b["bytes_rep"]
-    for x, y in zip(a["images"], b["images"]):
-        assert np.array_equal(x, y)
+    return cluster_script(oracle, n, stream, 1 << 20, 5)
+
+
+CLUSTER_SIZES = [1, 3, 5, 7]
+
+
+@pytest.mark.parametrize("n", CLUSTER_SIZES)
+def test_cluster_steps_match(orc, n):
+    b = observe_cluster_steps(orc, n)
+    assert digest(b) == reference(f"cluster_steps/{n}")
     # invariants of SURVEY.md s8a: commit == end on the leader at quiescence,
     # apply order == log order, every follower applied the same sequence
-    assert a["offsets"][0]["commit"] == a["offsets"][0]["end"]
-    idxs = [t[0] for t in a["applied"][0]]
+    assert b["offsets"][0]["commit"] == b["offsets"][0]["end"]
+    idxs = [t[0] for t in b["applied"][0]]
     assert idxs == sorted(idxs)
     for i in range(1, n):
-        assert a["applied"][i] == a["applied"][0]
+        assert b["applied"][i] == b["applied"][0]
 
 
-def test_cluster_wrap_and_prune_match(ref, orc):
+def observe_cluster_wrap_and_prune(oracle):
     """Ring of 16 KiB, pruning by HEAD entries between rounds, several laps."""
-    orc.set_rules(O.RULES_REFERENCE)
+    oracle.set_rules(O.RULES_REFERENCE)
     stream = S.ragged_stream(900, 150, conns=2, seed=77)
+    c = O.Cluster(oracle, 3, leader=0, term=1, length=16384)
+    c.prologue()
+    heads = []
+    cido = [(O.u64)(0) for _ in range(3)]
+    for k, (typ, clt, rid, payload) in enumerate(stream):
+        c.submit(typ, clt, rid, O.cmd_image(payload))
+        if k % 5 == 4:
+            c.round()
+            heads.append(c.prune())
+            c.round()
+            for i in (1, 2):
+                c.poll_head(i, cido[i])
+    c.round()
+    obs = dict(offsets=[c.offsets(i) for i in range(3)], images=[c.image(i) for i in range(3)],
+               applied=[c.applied(i) for i in range(3)], heads=heads)
+    c.close()
+    return obs
 
-    def run(oracle):
-        c = O.Cluster(oracle, 3, leader=0, term=1, length=16384)
-        c.prologue()
-        heads = []
-        cido = [(O.u64)(0) for _ in range(3)]
-        for k, (typ, clt, rid, payload) in enumerate(stream):
-            c.submit(typ, clt, rid, O.cmd_image(payload))
-            if k % 5 == 4:
-                c.round()
-                heads.append(c.prune())
-                c.round()
-                for i in (1, 2):
-                    c.poll_head(i, cido[i])
-        c.round()
-        obs = ([c.offsets(i) for i in range(3)], [c.image(i) for i in range(3)],
-               [c.applied(i) for i in range(3)], heads)
-        c.close()
-        return obs
 
-    a, b = run(ref), run(orc)
-    assert a[0] == b[0] and a[2] == b[2] and a[3] == b[3]
-    for x, y in zip(a[1], b[1]):
-        assert np.array_equal(x, y)
-    assert any(h for h in a[3])
+def test_cluster_wrap_and_prune_match(orc):
+    b = observe_cluster_wrap_and_prune(orc)
+    assert digest(b) == reference("cluster_wrap_and_prune")
+    assert any(h for h in b["heads"])
+
+
+def record(ref):
+    """Every observation above, made on the compiled reference (tests/golden/gen_golden.py)."""
+    out = {"layout": observe_layout(ref), "kat": observe_kat(ref),
+           "wrap_into_head_zero": observe_wrap_into_head_zero(ref),
+           "cluster_wrap_and_prune": observe_cluster_wrap_and_prune(ref)}
+    for seed, length in RANDOM_STREAMS:
+        out[f"random_stream/{seed}/{length}"] = observe_random_stream(ref, seed, length)
+    for left in WRAP_LEFT:
+        for typ in WRAP_TYPES:
+            out[f"wrap_edge/{left}/{typ}"] = observe_wrap_edge(ref, left, typ)
+    for n in CLUSTER_SIZES:
+        out[f"cluster_steps/{n}"] = observe_cluster_steps(ref, n)
+    return digest(out)

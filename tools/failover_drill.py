@@ -85,7 +85,15 @@ def run(n=5, nconn=4, nreq2=2000, plen=64, kill_after_s=1.0, spread=False, hb_us
             else:
                 missing.append(i)
         if lead["idx"] not in res:
-            raise RuntimeError(f"the new leader p{lead['idx']} produced no result")
+            p = procs[lead["idx"]]
+            state = "still running" if p.poll() is None else f"exit code {p.returncode}"
+            if p.poll() is None:
+                p.kill()
+            log = os.path.join(d, f"dare{lead['idx']}.log")
+            raise RuntimeError(f"the new leader p{lead['idx']} produced no result ({state}; progress "
+                               f"{open(p2).read().strip() if os.path.exists(p2) else 'none'}); its output:\n"
+                               + (p.communicate()[0] or b"").decode(errors="replace")[-2000:]
+                               + "\nits log:\n" + (open(log).read()[-3000:] if os.path.exists(log) else "absent"))
         logs = {i: open(os.path.join(d, f"dare{i}.log")).read() for i in range(n) if os.path.exists(os.path.join(d, f"dare{i}.log"))}
         out.update(new_leader=lead["idx"], term=lead["term"], requests_before_kill=before,
                    recovery_ms_kill_to_leader_line=round((lead["t_leader"] - t_kill) * 1e3, 2),
